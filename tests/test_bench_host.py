@@ -1,5 +1,5 @@
 """Host-side pieces of bench.py that do not need a GPU: the read generators (SURVEY §8(d) config 2: 0.2 %
-substitutions, 0.02 % indels), the stage -> kernel attribution of the roofline, the usable-CPU count."""
+substitutions, 0.02 % indels), the stage -> kernel attribution of the roofline, the usable-CPU count, the output dump."""
 import sys
 from pathlib import Path
 
@@ -40,3 +40,30 @@ def test_align_stage_split_names_the_seed_kernel_as_dominant(tmp_path):
 def test_usable_cpus_is_positive():
     n, note = bench.usable_cpus()
     assert n >= 1 and isinstance(note, str)
+
+
+def test_dump_outputs_writes_the_sampled_records_dereferenced(tmp_path):
+    """--dump-outputs: float64 arrays whose mappings and edits, split by n_mappings / n_edits, are each sampled read's path."""
+    g = synth.make_variant_graph(length=20000, n_snp=30, n_ins=4, n_del=4, n_haps=4, seed=9)
+    index = g.build_index()
+    rs = synth.simulate_pairs(g, 40, sub_rate=0.01, seed=5, indel_rate=0.002)
+    aln, maps, edits, status, _ = H.oracle_map_paired(index, rs.reads, rs.quals, H.paired_params(), threads=2)
+    idx = np.array([0, 3, 4, 17, 79])
+    bench.dump_outputs(tmp_path, idx, aln[idx], status[idx], aln[idx]["mapping_off"], aln[idx]["edit_off"],
+                       lambda i: maps[i], lambda i: edits[i])
+    got = {p.stem: np.load(p) for p in tmp_path.glob("*.npy")}
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert got["read_index"].tolist() == idx.tolist() and got["aln_score"].tolist() == aln[idx]["score"].tolist()
+    m = e = 0
+    for r, i in enumerate(idx):
+        _, _, path = H.decode_alignment(aln[i], maps, edits)
+        nm, ne = int(got["aln_n_mappings"][r]), int(got["aln_n_edits"][r])
+        assert got["mapping_node"][m: m + nm].tolist() == [n for n, _, _ in path]
+        assert got["mapping_offset"][m: m + nm].tolist() == [o for _, o, _ in path]
+        assert got["edits"][e: e + ne].tolist() == edits[int(aln[i]["edit_off"]): int(aln[i]["edit_off"]) + ne].tolist()
+        m, e = m + nm, e + ne
+    assert m == len(got["mapping_node"]) and e == len(got["edits"]) and m > 0 and e > 0
+    # the sample is fixed: the same reads whatever the run
+    s = bench.dump_sample(10_000_000)
+    assert len(s) == bench.DUMP_READS and (np.diff(s) > 0).all() and (s == bench.dump_sample(10_000_000)).all()
+    assert bench.dump_sample(100).tolist() == list(range(100))
